@@ -109,6 +109,69 @@ def raycast_replay(kind):
     return out
 
 
+def mixed_replay(kind):
+    """32^3 grid, 5 rounds of 5000 SetOccupancy events (seed 5), a local update box in round 3, then batch queries and the
+    sentinel returns (ESDFMap.cpp:402-410)."""
+    rng = np.random.default_rng(5)
+    m = pyoracle.OracleMap((-1.6, -1.6, -1.6), 0.1, (3.15, 3.15, 3.15), kind)
+    m.SetParameters(*scenes.PARAMS_TOGGLE)
+    out = {"grid_size": list(m.grid_size), "rounds": []}
+    for r in range(5):
+        n = 5000
+        vox = rng.integers(0, m.grid_size[0], (n, 3)).astype(np.int32)
+        occ = (rng.random(n) < 0.1).astype(np.uint8)
+        idx = m.SetOccupancyBatchVox(vox, occ)
+        if r == 3:   # local update box
+            m.SetUpdateRange((-1.0, -1.0, -1.0), (1.0, 0.8, 0.6))
+        changed = m.UpdateOccupancy(r != 3)
+        m.UpdateESDF()
+        c = checkpoint(m)
+        c.update(set_occupancy_returns_sha256=digest(idx), update_occupancy=bool(changed), stats=m.stats())
+        out["rounds"].append(c)
+        if r == 3:
+            m.SetOriginalRange()
+    pos = rng.uniform(-1.8, 1.8, (3000, 3))
+    d, g = m.GetDistWithGradTrilinearBatch(pos * 0.8)
+    out.update(distance_batch_sha256=digest(m.GetDistanceBatch(pos)), trilinear_dist_sha256=digest(d), trilinear_grad_sha256=digest(g),
+               sentinel_set_occupancy_bad_value=m.SetOccupancy((0.0, 0.0, 0.0), 2),
+               sentinel_set_occupancy_out_of_map=m.SetOccupancy((9.0, 0.0, 0.0), 1),
+               sentinel_get_distance_out_of_map=m.GetDistance((9.0, 0.0, 0.0)),
+               sentinel_trilinear_out_of_map=m.GetDistWithGradTrilinear((9.0, 0.0, 0.0))[0])
+    return out
+
+
+VIS_MAP = ((-3.2, -3.2, -1.6), 0.1, (6.4, 6.4, 3.2))
+
+
+def vis_replay(m):
+    """GetPointCloud / GetSliceMarker of map `m` (built with VIS_MAP) after 4 depth frames (seed 5/6), then inside a local
+    visualisation box (Fiesta.h:150).  Takes the map so the GPU test can drive the CUDA path through the same sequence."""
+    m.SetParameters(*scenes.PARAMS_DEFAULT)
+    sc = scenes.Scene((2.8, 2.8, 1.4), 8, 2, seed=5, edge=(0.3, 0.8))
+    for p, yaw in scenes.pose_walk(4, seed=6, clamp=0.5):
+        pts, T = scenes.depth_frame(sc, p, yaw, width=160, height=120, scale=0.25)
+        m.RaycastFrame(pts, T, 0.3, 4.0)
+        m.UpdateOccupancy(True)
+        m.UpdateESDF()
+        sc.step()
+
+    def cloud(lo, hi):
+        a = m.GetPointCloud(lo, hi)
+        return dict(n=len(a), sha256=digest(a))
+
+    def marker(sl, max_dist):
+        xyz, rgba = m.GetSliceMarker(sl, max_dist)
+        return dict(n=len(xyz), xyz_sha256=digest(xyz), rgba_sha256=digest(rgba))
+
+    out = {"point_cloud_0_31": cloud(0, 31), "point_cloud_10_20": cloud(10, 20)}
+    for sl in (0, 12, 16, 31):
+        out["slice_%d_2.0" % sl] = marker(sl, 2.0)
+    m.SetUpdateRange((-1.0, -1.5, -0.5), (2.0, 1.0, 0.7), False)
+    out["local_point_cloud_0_31"] = cloud(0, 31)
+    out["local_slice_14_1.0"] = marker(14, 1.0)
+    return out
+
+
 def dda_vectors(kind):
     """Raycast() known answers, including SURVEY.md Appendix B cases."""
     cases = [((1.5, 1.5, 1.5), (6.2, 3.7, 1.9)), ((6.2, 3.7, 1.9), (1.5, 1.5, 1.5)), ((2.0, 2.0, 2.0), (5.0, 5.0, 5.0)),
@@ -124,7 +187,8 @@ if __name__ == "__main__":
     assert pyoracle.available("ref"), "oracle/_ref is not built: run `make -C oracle ref` where /root/reference exists"
     gold = dict(generator="tests/golden/make_golden.py", source="oracle/_ref (unmodified reference ESDFMap.cpp + raycast.cpp)",
                 pillar_replay=pillar_replay("ref"), random_replay=random_replay("ref"), raycast_replay=raycast_replay("ref"),
-                dda=dda_vectors("ref"))
+                dda=dda_vectors("ref"), mixed_replay=mixed_replay("ref"),
+                vis_replay=vis_replay(pyoracle.OracleMap(*VIS_MAP, kind="ref")))
     with open(os.path.join(HERE, "reference_golden.json"), "w") as f:
         json.dump(gold, f, indent=1, sort_keys=True)
     print("wrote", os.path.join(HERE, "reference_golden.json"))
