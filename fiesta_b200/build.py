@@ -8,7 +8,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libfiesta_b200.so")
 SOURCES = ["fb_map.cu", "fb_esdf.cu", "fb_raycast.cu", "fb_exact.cu", "fb_xrelax.cu", "fb_vis.cu", "fb_depth.cu"]
-HEADERS = ["fb_common.cuh", "fb_exact.h", "fb_divmagic.h", os.path.join("..", "..", "include", "fiesta_b200.h")]
+HEADERS = ["fb_common.cuh", "fb_exact.h", "fb_divmagic.h", "fb_buf.h", os.path.join("..", "..", "include", "fiesta_b200.h")]
 # -fmad=false: the ray-casting, query and occupancy code must round every fp64 operation exactly like the reference's
 # separate multiply and add (ESDFMap.cpp:122-123, 519-537; raycast.cpp:100-107).
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-fmad=false", "-std=c++17",

@@ -19,6 +19,7 @@
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "fb_buf.h"
 
 #define FB_UNKNOWN 0u
 #define FB_INF 1u
@@ -207,4 +208,4 @@ struct FbDepthRel { double m[16]; };
 struct fiesta_depth_params;
 cudaError_t fb_depth_to_cloud(const uint16_t *d_img, const uint16_t *d_last, int rows, int cols, const fiesta_depth_params &p, int filter_on,
                               const FbDepthRel &rel, float *d_pts, uint8_t *d_flags, uint32_t *d_sel, float *d_cloud, unsigned *d_count,
-                              void **tmp, size_t *tmp_bytes, unsigned *h_n, cudaStream_t s);
+                              FbDev<uint8_t> &tmp, unsigned *h_n, cudaStream_t s);

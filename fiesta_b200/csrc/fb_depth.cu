@@ -44,15 +44,15 @@ __global__ void k_depth_gather(const float *pts, const uint32_t *sel, unsigned n
 // d_sel rows*cols u32.  Returns the number of points in d_cloud (pixel order).
 cudaError_t fb_depth_to_cloud(const uint16_t *d_img, const uint16_t *d_last, int rows, int cols, const fiesta_depth_params &p, int filter_on,
                               const FbDepthRel &rel, float *d_pts, uint8_t *d_flags, uint32_t *d_sel, float *d_cloud, unsigned *d_count,
-                              void **tmp, size_t *tmp_bytes, unsigned *h_n, cudaStream_t s) {
+                              FbDev<uint8_t> &tmp, unsigned *h_n, cudaStream_t s) {
   const size_t N = (size_t)rows * cols;
   k_depth_project<<<(unsigned)((N + 255) / 256), 256, 0, s>>>(d_img, d_last, rows, cols, p, filter_on, rel, d_pts, d_flags);
   thrust::counting_iterator<uint32_t> it(0);
   size_t bytes = 0;
   cudaError_t e = cub::DeviceSelect::Flagged(nullptr, bytes, it, d_flags, d_sel, d_count, (int)N, s);
   if (e) return e;
-  if (bytes > *tmp_bytes) { if (*tmp) cudaFree(*tmp); *tmp_bytes = bytes + (1u << 20); if ((e = cudaMalloc(tmp, *tmp_bytes))) return e; }
-  if ((e = cub::DeviceSelect::Flagged(*tmp, bytes, it, d_flags, d_sel, d_count, (int)N, s))) return e;
+  if ((e = tmp.reserve(bytes, s, false))) return e;
+  if ((e = cub::DeviceSelect::Flagged(tmp.get(), bytes, it, d_flags, d_sel, d_count, (int)N, s))) return e;
   if ((e = cudaMemcpyAsync(h_n, d_count, 4, cudaMemcpyDeviceToHost, s))) return e;
   if ((e = cudaStreamSynchronize(s))) return e;
   if (*h_n) k_depth_gather<<<(*h_n + 255) / 256, 256, 0, s>>>(d_pts, d_sel, *h_n, d_cloud);

@@ -21,6 +21,7 @@
 #include <cub/cub.cuh>
 #include <stdio.h>
 #include <stdlib.h>
+#include <algorithm>
 #include <chrono>
 #include "fb_common.cuh"
 #include "fb_exact.h"
@@ -114,31 +115,14 @@ __global__ void k_x_fill64(unsigned long long *a, size_t n, unsigned long long v
 #define XCK(call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) { snprintf(X->err, sizeof(X->err), "%s: %s", #call, cudaGetErrorString(e__)); return e__; } } while (0)
 static inline unsigned nblk(size_t n, unsigned t = 256) { return (unsigned)((n + t - 1) / t); }
 
-template <typename T>
-static cudaError_t x_ensure(FbExact *X, T **p, size_t *cap, size_t need) {
-  if (need <= *cap) return cudaSuccess;
-  size_t nc = need + need / 2 + 4096;
-  T *np = nullptr;
-  XCK(cudaMalloc((void **)&np, nc * sizeof(T)));
-  if (*p) cudaFree(*p);
-  *p = np; *cap = nc;
-  return cudaSuccess;
-}
-static cudaError_t x_tmp(FbExact *X, size_t bytes) {
-  if (bytes <= X->cub_bytes) return cudaSuccess;
-  if (X->cub_tmp) cudaFree(X->cub_tmp);
-  X->cub_bytes = bytes + bytes / 2 + (1u << 20);
-  XCK(cudaMalloc(&X->cub_tmp, X->cub_bytes));
-  return cudaSuccess;
-}
 // ordered compaction: out[0..count) = in[i] for flags[i] != 0, order kept
 static cudaError_t x_select(FbExact *X, const uint32_t *in, const uint8_t *flags, uint32_t *out, unsigned n, unsigned *count, cudaStream_t s) {
   *count = 0;
   if (n == 0) return cudaSuccess;
   size_t bytes = 0;
-  XCK(cub::DeviceSelect::Flagged(nullptr, bytes, in, flags, out, X->d_count, (int)n, s));
-  cudaError_t e = x_tmp(X, bytes); if (e) return e;
-  XCK(cub::DeviceSelect::Flagged(X->cub_tmp, bytes, in, flags, out, X->d_count, (int)n, s));
+  XCK(cub::DeviceSelect::Flagged(nullptr, bytes, in, flags, out, X->d_count.get(), (int)n, s));
+  XCK(X->cub_tmp.reserve(bytes, s, false));
+  XCK(cub::DeviceSelect::Flagged(X->cub_tmp.get(), bytes, in, flags, out, X->d_count.get(), (int)n, s));
   XCK(cudaMemcpyAsync(X->h_count, X->d_count, 4, cudaMemcpyDeviceToHost, s));
   XCK(cudaStreamSynchronize(s));
   *count = *X->h_count;
@@ -148,85 +132,59 @@ static cudaError_t x_sort_pairs(FbExact *X, const unsigned long long *kin, unsig
                                 int key_bits = 64) {
   size_t bytes = 0;
   XCK(cub::DeviceRadixSort::SortPairs(nullptr, bytes, kin, kout, vin, vout, (int)n, 0, key_bits, s));
-  cudaError_t e = x_tmp(X, bytes); if (e) return e;
-  XCK(cub::DeviceRadixSort::SortPairs(X->cub_tmp, bytes, kin, kout, vin, vout, (int)n, 0, key_bits, s));
+  XCK(X->cub_tmp.reserve(bytes, s, false));
+  XCK(cub::DeviceRadixSort::SortPairs(X->cub_tmp.get(), bytes, kin, kout, vin, vout, (int)n, 0, key_bits, s));
   return cudaSuccess;
 }
 cudaError_t fb_exact_init(FbExact *X, const FbGeom &g, int device, cudaStream_t s) {
-  memset(X, 0, sizeof(*X));
   const size_t P = (size_t)g.ptotal;
   XCK(fb_xrelax_init());
   X->relax_blocks = fb_xrelax_blocks(device);
   if (X->relax_blocks <= 0 || X->relax_blocks > FB_X_MAX_BLOCKS) { snprintf(X->err, sizeof(X->err), "k_x_relax does not fit on this device"); return cudaErrorInvalidConfiguration; }
-  XCK(cudaMalloc((void **)&X->MB, P * 8)); XCK(cudaMalloc((void **)&X->LS, P * 8)); XCK(cudaMalloc((void **)&X->tkey, P * 8));
-  XCK(cudaMalloc((void **)&X->touched, P * 4));
-  XCK(cudaMalloc((void **)&X->SUM, P * 16)); XCK(cudaMalloc((void **)&X->SUMg, P * 4)); XCK(cudaMemsetAsync(X->SUMg, 0, P * 4, s));
-  XCK(cudaMalloc((void **)&X->emask, P * 4));
-  XCK(cudaMalloc((void **)&X->wstamp, P * 4)); XCK(cudaMemsetAsync(X->wstamp, 0, P * 4, s));
-  for (int k = 0; k < 3; ++k) { XCK(cudaMalloc((void **)&X->W[k], P * 4)); XCK(cudaMalloc((void **)&X->F[k], P * 4)); }
-  for (int k = 0; k < 2; ++k) { XCK(cudaMalloc((void **)&X->E[k], P * 4)); X->cap_E[k] = P; }
+  XCK(X->MB.alloc(P)); XCK(X->LS.alloc(P)); XCK(X->tkey.alloc(P));
+  XCK(X->touched.alloc(P));
+  XCK(X->SUM.alloc(P)); XCK(X->SUMg.alloc(P)); XCK(cudaMemsetAsync(X->SUMg, 0, P * 4, s));
+  XCK(X->emask.alloc(P));
+  XCK(X->wstamp.alloc(P)); XCK(cudaMemsetAsync(X->wstamp, 0, P * 4, s));
+  for (int k = 0; k < 3; ++k) { XCK(X->W[k].alloc(P)); XCK(X->F[k].alloc(P)); }
+  for (int k = 0; k < 2; ++k) XCK(X->E[k].alloc(P));
   X->dense_min = 16384u;
   if (const char *e = getenv("FIESTA_X_DENSE")) { long v = atol(e); if (v >= 0 && v <= (1 << 24)) X->dense_min = (unsigned)v; }
   X->small_max = FB_X_SMALL_DEFAULT;
   if (const char *e = getenv("FIESTA_X_SMALL")) { long v = atol(e); if (v >= 0 && v <= 65536) X->small_max = (unsigned)v; }
-  XCK(cudaMalloc((void **)&X->slotc, ((size_t)X->small_max + 1) * 32 * 4));
+  XCK(X->slotc.alloc(((size_t)X->small_max + 1) * 32));
   // Per-frame work arrays (touched voxels, dependants of deleted obstacles, sort scratch) are sized up front for 1/8 of the
-  // grid: growing them on demand puts cudaMalloc / cudaFree (device-wide synchronisations, milliseconds) inside UpdateESDF.
-  {
-    const size_t c0 = P / 8 > (1u << 20) ? P / 8 : (1u << 20);
-    cudaError_t e;
-    if ((e = x_ensure(X, &X->k1, &X->cap_k1, c0)) || (e = x_ensure(X, &X->k2, &X->cap_k2, c0)) || (e = x_ensure(X, &X->k1b, &X->cap_k1b, c0)) ||
-        (e = x_ensure(X, &X->k2b, &X->cap_k2b, c0)) || (e = x_ensure(X, &X->dv, &X->cap_dv, c0)) || (e = x_ensure(X, &X->idx[0], &X->cap_idx[0], c0)) ||
-        (e = x_ensure(X, &X->idx[1], &X->cap_idx[1], c0)) || (e = x_ensure(X, &X->deps, &X->cap_deps, c0)) || (e = x_ensure(X, &X->nc[0], &X->cap_nc[0], c0)) ||
-        (e = x_ensure(X, &X->nc[1], &X->cap_nc[1], c0)) || (e = x_ensure(X, &X->flags, &X->cap_flags, c0)) || (e = x_ensure(X, &X->flags2, &X->cap_flags2, c0)) ||
-        (e = x_ensure(X, &X->sel, &X->cap_sel, c0)) || (e = x_tmp(X, c0 * 16 + (64u << 20)))) return e;
-  }
-  XCK(cudaMalloc((void **)&X->d_ctl, sizeof(FbXCtl))); XCK(cudaMemsetAsync(X->d_ctl, 0, sizeof(FbXCtl), s));
-  XCK(cudaMallocHost((void **)&X->h_ctl, sizeof(FbXCtl)));
-  XCK(cudaMalloc((void **)&X->d_count, 16)); XCK(cudaMalloc((void **)&X->d_flag, 16));
-  XCK(cudaMallocHost((void **)&X->h_count, 16));
-  XCK(cudaMemsetAsync(X->d_count, 0, 16, s)); XCK(cudaMemsetAsync(X->d_flag, 0, 16, s));
+  // grid: growing them on demand puts an allocation and a free (device-wide synchronisations, milliseconds) inside UpdateESDF.
+  const size_t c0 = P / 8 > (1u << 20) ? P / 8 : (1u << 20);
+  for (FbDev<unsigned long long> *b : {&X->k1, &X->k2, &X->k1b, &X->k2b}) XCK(b->reserve(c0, s, false));
+  for (FbDev<uint32_t> *b : {&X->dv, &X->idx[0], &X->idx[1], &X->deps, &X->nc[0], &X->nc[1], &X->sel}) XCK(b->reserve(c0, s, false));
+  XCK(X->flags.reserve(c0, s, false)); XCK(X->flags2.reserve(c0, s, false));
+  XCK(X->cub_tmp.reserve(c0 * 16 + (64u << 20), s, false));
+  XCK(X->d_ctl.alloc(1)); XCK(cudaMemsetAsync(X->d_ctl, 0, sizeof(FbXCtl), s));
+  XCK(X->h_ctl.alloc(1));
+  XCK(X->d_count.alloc(4)); XCK(X->h_count.alloc(4));
+  XCK(cudaMemsetAsync(X->d_count, 0, 16, s));
   k_x_fill64<<<148 * 8, 256, 0, s>>>(X->MB, P, XMB_NONE);
   XCK(cudaMemsetAsync(X->tkey, 0, P * 8, s));
   XCK(cudaMemsetAsync(X->LS, 0, P * 8, s));
   X->tclock = 1; X->key_base = 0; X->key_epoch = 1; X->key_hi = 1ull << FB_KEY_BITS; X->gen_id = 0; X->wclock = 0; X->sclock = 0;
   return cudaGetLastError();
 }
-void fb_exact_free(FbExact *X) {
-  void *p[] = {X->MB, X->LS, X->tkey, X->touched, X->SUM, X->SUMg, X->emask, X->wstamp, X->W[0], X->W[1], X->W[2], X->F[0], X->F[1], X->F[2], X->slotc,
-               X->d_ctl, X->d_dbg, X->d_count, X->d_flag, X->E[0], X->E[1], X->sel,
-               X->k1, X->k2, X->k1b, X->k2b, X->dv, X->idx[0], X->idx[1], X->deps, X->nc[0], X->nc[1], X->flags, X->flags2, X->cub_tmp};
-  for (void *q : p) if (q) cudaFree(q);
-  if (X->h_count) cudaFreeHost(X->h_count);
-  if (X->h_ctl) cudaFreeHost(X->h_ctl);
-  memset(X, 0, sizeof(*X));
-}
-
 // Second half of UpdateOccupancy (ESDFMap.cpp:263-267): k_integrate<true> (fb_map.cu) staged the voxels that crossed the
 // occupancy threshold with the serial time of their first observation; sorted by that time they are appended to
 // insert_queue_ / delete_queue_ in the order the reference's walk over occupancy_queue_ pushes them.
 cudaError_t fb_exact_queue_crossings(FbExact *X, const unsigned long long *ins_key, const uint32_t *ins_vox, const unsigned long long *del_key,
-                                     const uint32_t *del_vox, uint32_t **ins, size_t *cap_ins, unsigned *n_ins, uint32_t **del, size_t *cap_del,
-                                     unsigned *n_del, cudaStream_t s, int *launches) {
+                                     const uint32_t *del_vox, FbDev<uint32_t> &ins, unsigned *n_ins, FbDev<uint32_t> &del, unsigned *n_del,
+                                     cudaStream_t s, int *launches) {
   cudaError_t e;
   XCK(cudaMemcpyAsync(X->h_count, X->d_count, 8, cudaMemcpyDeviceToHost, s));
   XCK(cudaStreamSynchronize(s));
   const unsigned ni = X->h_count[0], nd = X->h_count[1];
-  for (int q = 0; q < 2; ++q) {                                 // grow the queues if needed (contents kept)
-    uint32_t **lst = q ? del : ins; size_t *cap = q ? cap_del : cap_ins; const unsigned have = q ? *n_del : *n_ins, add = q ? nd : ni;
-    if ((size_t)have + add > *cap) {
-      size_t nc = (size_t)have + add + ((size_t)have + add) / 2 + 4096;
-      uint32_t *np = nullptr;
-      XCK(cudaMalloc((void **)&np, nc * 4));
-      if (*lst && have) XCK(cudaMemcpyAsync(np, *lst, (size_t)have * 4, cudaMemcpyDeviceToDevice, s));
-      XCK(cudaStreamSynchronize(s));
-      if (*lst) cudaFree(*lst);
-      *lst = np; *cap = nc;
-    }
-  }
-  if ((e = x_ensure(X, &X->k1b, &X->cap_k1b, ni > nd ? ni : nd))) return e;
-  if (ni) { if ((e = x_sort_pairs(X, ins_key, X->k1b, ins_vox, *ins + *n_ins, ni, s, FB_KEY_BITS))) return e; *n_ins += ni; *launches += 1; }
-  if (nd) { if ((e = x_sort_pairs(X, del_key, X->k1b, del_vox, *del + *n_del, nd, s, FB_KEY_BITS))) return e; *n_del += nd; *launches += 1; }
+  XCK(ins.reserve((size_t)*n_ins + ni, s, true));             // the queues keep the pushes of an earlier UpdateOccupancy
+  XCK(del.reserve((size_t)*n_del + nd, s, true));
+  XCK(X->k1b.reserve(ni > nd ? ni : nd, s, false));
+  if (ni) { if ((e = x_sort_pairs(X, ins_key, X->k1b, ins_vox, ins + *n_ins, ni, s, FB_KEY_BITS))) return e; *n_ins += ni; *launches += 1; }
+  if (nd) { if ((e = x_sort_pairs(X, del_key, X->k1b, del_vox, del + *n_del, nd, s, FB_KEY_BITS))) return e; *n_del += nd; *launches += 1; }
   return cudaSuccess;
 }
 // A new integration epoch: later observations beat everything recorded so far in tkey (fb_touch), so nothing is reset.
@@ -245,7 +203,7 @@ cudaError_t fb_exact_update_esdf(FbExact *X, const FbGeom &g, uint32_t *cobs, ui
   cudaError_t e;
   const size_t P = (size_t)g.ptotal;
   memset(st, 0, sizeof(*st));
-  if ((e = x_ensure(X, &X->flags, &X->cap_flags, (size_t)(n_ins > n_del ? n_ins : n_del) + 16))) return e;
+  XCK(X->flags.reserve((size_t)(n_ins > n_del ? n_ins : n_del) + 16, s, false));
   static const bool xdbg = getenv("FIESTA_DEBUG_X") != nullptr;
   auto now = [] { return std::chrono::steady_clock::now(); };
   auto ms = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) { return std::chrono::duration<double, std::milli>(b - a).count(); };
@@ -263,7 +221,7 @@ cudaError_t fb_exact_update_esdf(FbExact *X, const FbGeom &g, uint32_t *cobs, ui
   }
   // ---- E2: deletes (:292-337)
   if (n_del) {
-    if ((e = x_ensure(X, &X->sel, &X->cap_sel, (size_t)n_del + 16))) return e;
+    XCK(X->sel.reserve((size_t)n_del + 16, s, false));
     // `scratch` (one word per voxel) is all-XNONE between uses: every sparse use below undoes its own writes instead of
     // refilling 4 bytes per voxel of the grid three times per call
     if (!X->scratch_clean) { k_x_fill32<<<148 * 8, 256, 0, s>>>(scratch, P, XNONE); *launches += 1; }
@@ -286,29 +244,22 @@ cudaError_t fb_exact_update_esdf(FbExact *X, const FbGeom &g, uint32_t *cobs, ui
       // dependants: the list is sized by a first counting attempt, then (rarely) re-run with more room
       unsigned ndep = 0;
       for (int attempt = 0; attempt < 2; ++attempt) {
-        size_t cap = X->cap_dv;
+        const size_t cap = std::min({X->dv.size(), X->k1.size(), X->k2.size()});
         XCK(cudaMemsetAsync(X->d_count, 0, 4, s));
-        k_x_scan_deps<<<148 * 16, 256, 0, s>>>(g, cobs, occbits, scratch, X->LS, X->k1, X->k2, X->dv, X->d_count, (unsigned)((cap < X->cap_k1 ? cap : X->cap_k1) < X->cap_k2 ? (cap < X->cap_k1 ? cap : X->cap_k1) : X->cap_k2), shift);
+        k_x_scan_deps<<<148 * 16, 256, 0, s>>>(g, cobs, occbits, scratch, X->LS, X->k1, X->k2, X->dv, X->d_count, (unsigned)cap, shift);
         XCK(cudaMemcpyAsync(X->h_count, X->d_count, 4, cudaMemcpyDeviceToHost, s));
         XCK(cudaStreamSynchronize(s));
         ndep = *X->h_count;
         *launches += 1;
-        if (ndep <= cap && ndep <= X->cap_k1 && ndep <= X->cap_k2) break;
-        if ((e = x_ensure(X, &X->dv, &X->cap_dv, ndep))) return e;
-        if ((e = x_ensure(X, &X->k1, &X->cap_k1, ndep))) return e;
-        if ((e = x_ensure(X, &X->k2, &X->cap_k2, ndep))) return e;
+        if (ndep <= cap) break;
+        XCK(X->dv.reserve(ndep, s, false)); XCK(X->k1.reserve(ndep, s, false)); XCK(X->k2.reserve(ndep, s, false));
       }
       st->dependants = ndep;
       k_x_unset<<<nblk(nd), 256, 0, s>>>(X->sel, nd, scratch);
       if (ndep) {
-        if ((e = x_ensure(X, &X->k1b, &X->cap_k1b, ndep))) return e;
-        if ((e = x_ensure(X, &X->k2b, &X->cap_k2b, ndep))) return e;
-        if ((e = x_ensure(X, &X->idx[0], &X->cap_idx[0], ndep))) return e;
-        if ((e = x_ensure(X, &X->idx[1], &X->cap_idx[1], ndep))) return e;
-        if ((e = x_ensure(X, &X->deps, &X->cap_deps, ndep))) return e;
-        if ((e = x_ensure(X, &X->nc[0], &X->cap_nc[0], ndep))) return e;
-        if ((e = x_ensure(X, &X->nc[1], &X->cap_nc[1], ndep))) return e;
-        if ((e = x_ensure(X, &X->flags, &X->cap_flags, ndep))) return e;
+        for (FbDev<unsigned long long> *b : {&X->k1b, &X->k2b}) XCK(b->reserve(ndep, s, false));
+        for (FbDev<uint32_t> *b : {&X->idx[0], &X->idx[1], &X->deps, &X->nc[0], &X->nc[1]}) XCK(b->reserve(ndep, s, false));
+        XCK(X->flags.reserve(ndep, s, false));
         if (shift) {
           if ((e = x_sort_pairs(X, X->k1, X->k1b, X->dv, X->deps, ndep, s))) return e;
           *launches += 1;
@@ -320,7 +271,7 @@ cudaError_t fb_exact_update_esdf(FbExact *X, const FbGeom &g, uint32_t *cobs, ui
           k_x_gather32<<<nblk(ndep), 256, 0, s>>>(X->dv, X->idx[0], ndep, X->deps);
           *launches += 5;
         }
-        if ((e = x_ensure(X, &X->flags2, &X->cap_flags2, ndep))) return e;
+        XCK(X->flags2.reserve(ndep, s, false));
         k_x_set_ord<<<nblk(ndep), 256, 0, s>>>(X->deps, ndep, scratch, X->nc[0], X->flags2);
         *launches += 1;
         ndep_run = ndep; ls_deps = X->tclock;                // the fixpoint and the hand-over to E[0] run inside k_x_relax
@@ -332,7 +283,7 @@ cudaError_t fb_exact_update_esdf(FbExact *X, const FbGeom &g, uint32_t *cobs, ui
   st->generations = 0;
   if (xdbg) { cudaStreamSynchronize(s); fprintf(stderr, "[x] seeds+deletes %.2f ms (reseed rounds %u, dependants %u)\n", ms(t_begin, now()), st->reseed_rounds, st->dependants); }
   if (nE || ndep_run) {
-    if (xdbg && !X->d_dbg) XCK(cudaMalloc((void **)&X->d_dbg, FB_X_DBG_WORDS * 8));
+    if (xdbg && !X->d_dbg) XCK(X->d_dbg.alloc(FB_X_DBG_WORDS));
     if (xdbg) XCK(cudaMemsetAsync(X->d_dbg, 0, FB_X_DBG_WORDS * 8, s));
     if (X->sclock > 0xf0000000u) { XCK(cudaMemsetAsync(X->SUMg, 0, P * 4, s)); X->sclock = 0; }       // stamp wrap-around
     if (X->gen_id > 0xf0000000u) X->gen_id = 0;
@@ -341,7 +292,7 @@ cudaError_t fb_exact_update_esdf(FbExact *X, const FbGeom &g, uint32_t *cobs, ui
     memset(h, 0, sizeof(*h));
     h->gen_id = X->gen_id; h->wclock = X->wclock; h->tclock = X->tclock; h->sclock = X->sclock;
     XCK(cudaMemcpyAsync(X->d_ctl, h, sizeof(FbXCtl), cudaMemcpyHostToDevice, s));
-    XCK(fb_xrelax_launch(X, g, cobs, nE, X->deps, ndep_run, scratch, X->nc[0], X->flags2, occbits, ls_deps, xdbg ? X->d_dbg : nullptr, s));
+    XCK(fb_xrelax_launch(X, g, cobs, nE, X->deps, ndep_run, scratch, X->nc[0], X->flags2, occbits, ls_deps, xdbg ? X->d_dbg.get() : nullptr, s));
     if (ndep_run) k_x_unset<<<nblk(ndep_run), 256, 0, s>>>(X->deps, ndep_run, scratch);
     XCK(cudaMemcpyAsync(h, X->d_ctl, sizeof(FbXCtl), cudaMemcpyDeviceToHost, s));
     XCK(cudaStreamSynchronize(s));

@@ -25,42 +25,40 @@ struct FbXCtl {
 };
 
 struct FbExact {
-  unsigned long long *MB;      // per voxel: {parity | queue position | behaviour | code} of its live entry in the current generation
-  unsigned long long *LS;      // per voxel: time of the last relink into a dependant list
-  unsigned long long *tkey;    // per voxel: epoch-coded serial time of the first pending observation (fb_touch, fb_common.cuh)
-  uint32_t *touched;           // [ptotal] staging of the voxels whose occupancy crossed the threshold (inserts; deletes use emask)
+  FbDev<unsigned long long> MB;   // per voxel: {parity | queue position | behaviour | code} of its live entry in the current generation
+  FbDev<unsigned long long> LS;   // per voxel: time of the last relink into a dependant list
+  FbDev<unsigned long long> tkey; // per voxel: epoch-coded serial time of the first pending observation (fb_touch, fb_common.cuh)
+  FbDev<uint32_t> touched;     // [ptotal] staging of the voxels whose occupancy crossed the threshold (inserts; deletes use emask)
   unsigned long long tclock;   // relink clock
   unsigned long long key_base; // observation clock within the current integration epoch
   unsigned long long key_hi;   // key_epoch << FB_KEY_BITS
   unsigned key_epoch;          // integration epoch (one per UpdateOccupancy)
-  unsigned *d_count, *d_flag, *h_count;
+  FbDev<unsigned> d_count; FbPinned<unsigned> h_count;
   bool scratch_clean;           // the per-voxel scratch word array of UpdateESDF is all-XNONE
-  uint4 *SUM;                  // per voxel offer summary of the current generation: {first ts, best ts, best code, snapshot code}
-  uint32_t *SUMg;              // per voxel: summary pass for which SUM was computed (each target is claimed once per pass)
+  FbDev<uint4> SUM;            // per voxel offer summary of the current generation: {first ts, best ts, best code, snapshot code}
+  FbDev<uint32_t> SUMg;        // per voxel: summary pass for which SUM was computed (each target is claimed once per pass)
   unsigned gen_id, wclock, sclock;
-  uint32_t *emask;             // per entry: slots it owns in the next generation
-  uint32_t *W[3], *F[3];       // work lists / flip lists, rotating per round
-  uint32_t *wstamp;            // per entry: round for which it is already in a work list
-  uint32_t *slotc;             // SMALL generations: codes of the owned slots
+  FbDev<uint32_t> emask;       // per entry: slots it owns in the next generation
+  FbDev<uint32_t> W[3], F[3];  // work lists / flip lists, rotating per round
+  FbDev<uint32_t> wstamp;      // per entry: round for which it is already in a work list
+  FbDev<uint32_t> slotc;       // SMALL generations: codes of the owned slots
   unsigned dense_min;          // work lists longer than this are evaluated through refreshed summaries (one wave of warps)
   unsigned small_max;          // generations up to this many entries run without summaries
-  FbXCtl *d_ctl, *h_ctl;
-  unsigned long long *d_dbg;
+  FbDev<FbXCtl> d_ctl; FbPinned<FbXCtl> h_ctl;
+  FbDev<unsigned long long> d_dbg;
   int relax_blocks;
-  uint32_t *E[2]; size_t cap_E[2];
-  uint32_t *sel; size_t cap_sel;
-  unsigned long long *k1, *k2, *k1b, *k2b; size_t cap_k1, cap_k2, cap_k1b, cap_k2b;
-  uint32_t *dv, *idx[2], *deps, *nc[2]; size_t cap_dv, cap_idx[2], cap_deps, cap_nc[2];
-  uint8_t *flags, *flags2; size_t cap_flags, cap_flags2;
-  void *cub_tmp; size_t cub_bytes;
+  FbDev<uint32_t> E[2], sel;
+  FbDev<unsigned long long> k1, k2, k1b, k2b;
+  FbDev<uint32_t> dv, idx[2], deps, nc[2];
+  FbDev<uint8_t> flags, flags2;
+  FbDev<uint8_t> cub_tmp;
   char err[256];
 };
 
 cudaError_t fb_exact_init(FbExact *X, const FbGeom &g, int device, cudaStream_t s);
-void fb_exact_free(FbExact *X);
 cudaError_t fb_exact_queue_crossings(FbExact *X, const unsigned long long *ins_key, const uint32_t *ins_vox, const unsigned long long *del_key,
-                                     const uint32_t *del_vox, uint32_t **ins, size_t *cap_ins, unsigned *n_ins, uint32_t **del, size_t *cap_del,
-                                     unsigned *n_del, cudaStream_t s, int *launches);
+                                     const uint32_t *del_vox, FbDev<uint32_t> &ins, unsigned *n_ins, FbDev<uint32_t> &del, unsigned *n_del,
+                                     cudaStream_t s, int *launches);
 cudaError_t fb_exact_next_epoch(FbExact *X, const FbGeom &g, cudaStream_t s);
 cudaError_t fb_exact_update_esdf(FbExact *X, const FbGeom &g, uint32_t *cobs, uint32_t *scratch, const double *occ, const uint32_t *occbits, double l_occ,
                                  const uint32_t *ins, unsigned n_ins, const uint32_t *del, unsigned n_del, cudaStream_t s, FbExactStats *st, int *launches);

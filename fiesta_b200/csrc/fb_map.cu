@@ -8,6 +8,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <string>
+#include <memory>
 #include <new>
 #include "../../include/fiesta_b200.h"
 #include "fb_common.cuh"
@@ -33,44 +34,51 @@ struct fiesta_map {
   double l_hit, l_miss, l_min, l_max, l_occ;
   double l_cornor[3], r_cornor[3];
   // per-voxel state
-  uint32_t *cobs, *cobs_b, *stamp[2], *occbits;
-  double *occ;
-  unsigned long long *cnt;
+  FbDev<uint32_t> cobs, cobs_b, stamp[2], occbits;
+  FbDev<double> occ;
+  FbDev<unsigned long long> cnt;
   // tiles
-  uint32_t *tile_flag, *nb_flag, *list[2], *changed[2], *changed_bbox[2];
+  FbDev<uint32_t> tile_flag, nb_flag, list[2], changed[2], changed_bbox[2];
   CUtensorMap tmap;
   int wf_blocks, rr_blocks;
   // queues
-  uint32_t *touch_flag, *touch_list;
+  FbDev<uint32_t> touch_flag, touch_list;
   unsigned touch_epoch;
-  uint32_t *ins, *del;
-  size_t cap_ins, cap_del;
+  FbDev<uint32_t> ins, del;
   unsigned n_touch_tiles, n_ins, n_del;  // host view (valid after the last sync)
-  FbCounters *d_ctr, *h_ctr;
+  FbDev<FbCounters> d_ctr;
+  FbPinned<FbCounters> h_ctr;
   // per-call SetOccupancy staging
-  uint32_t *h_ev, *d_ev;
-  size_t n_ev, cap_ev;
+  FbPinned<uint32_t> h_ev;
+  FbDev<uint32_t> d_ev;
+  size_t n_ev;
   // ray casting
-  float *d_xyz; size_t cap_xyz;
-  uint32_t *ray_list; size_t cap_ray_list;
-  int *ray_len, *ray_reach; unsigned *ray_dirty; size_t cap_rays;
+  FbDev<float> d_xyz;
+  FbDev<uint32_t> ray_list;
+  FbDev<int> ray_len, ray_reach;
+  FbDev<unsigned> ray_dirty;
   unsigned frame_tag, owner_tag;
   // queries
-  double *d_qin, *d_qout; size_t cap_q;
+  FbDev<double> d_qin, d_qout;
   cudaEvent_t ev[4];
-  unsigned long long *d_dbg;
-  // depth front end (next #1)
-  uint16_t *d_img[2]; size_t cap_img; unsigned image_cnt;
-  float *d_dpts, *d_dcloud; uint8_t *d_dflags; uint32_t *d_dsel; unsigned *d_dcount; void *d_dtmp; size_t d_dtmp_bytes; unsigned last_cloud_n;
+  FbDev<unsigned long long> d_dbg;
+  // depth front end (next #1): sized exactly for cap_img pixels
+  FbDev<uint16_t> d_img[2]; size_t cap_img; unsigned image_cnt;
+  FbDev<float> d_dpts, d_dcloud; FbDev<uint8_t> d_dflags; FbDev<uint32_t> d_dsel; FbDev<unsigned> d_dcount; FbDev<uint8_t> d_dtmp; unsigned last_cloud_n;
   int mode;
   int shard_rank, shard_world, tile_x_lo, tile_x_hi;
-  unsigned *d_halo_changed;
+  FbDev<unsigned> d_halo_changed;
   FbExact X;
   fiesta_stats st;
   // pinned host mirror (next #3): union of the update boxes that were current while records could change
   struct fiesta_host_mirror *mirror;
   int dirty_lo[3], dirty_hi[3];
   bool dirty_any, pending_obs;      // pending_obs: observations counted under the current box and not integrated yet
+  // No constructor, so `new fiesta_map()` zero-fills every plain member.  The buffers free themselves after this body.
+  ~fiesta_map() {
+    for (cudaEvent_t e : ev) if (e) cudaEventDestroy(e);
+    if (stream) cudaStreamDestroy(stream);
+  }
 };
 static void mark_dirty(fiesta_map *m) {                                   // tracked without a mirror too: events staged before a mirror is
   const FbGeom &g = m->g;                                                   // created are integrated after it
@@ -315,17 +323,6 @@ static bool host_pos_in_map(const FbGeom &g, const double *p) {
 static void host_pos2vox(const FbGeom &g, const double *p, int *v) {
   for (int i = 0; i < 3; ++i) v[i] = (int)floor((p[i] - g.origin[i]) / g.res);
 }
-template <typename T>
-static int ensure(T **ptr, size_t *cap, size_t need, bool keep, cudaStream_t s) {
-  if (need <= *cap) return FIESTA_OK;
-  size_t ncap = need + need / 2 + 1024;
-  T *np = nullptr;
-  CK(cudaMalloc((void **)&np, ncap * sizeof(T)));
-  if (keep && *ptr && *cap) { CK(cudaMemcpyAsync(np, *ptr, *cap * sizeof(T), cudaMemcpyDeviceToDevice, s)); CK(cudaStreamSynchronize(s)); }
-  if (*ptr) cudaFree(*ptr);
-  *ptr = np; *cap = ncap;
-  return FIESTA_OK;
-}
 static int fetch_counters(fiesta_map *m) {
   CK(cudaMemcpyAsync(m->h_ctr, m->d_ctr, sizeof(FbCounters), cudaMemcpyDeviceToHost, m->stream));
   CK(cudaStreamSynchronize(m->stream));
@@ -337,7 +334,7 @@ static int flush_events(fiesta_map *m) {
   if (m->n_ev == 0) return FIESTA_OK;
   CK(cudaMemcpyAsync(m->d_ev, m->h_ev, m->n_ev * sizeof(uint32_t), cudaMemcpyHostToDevice, m->stream));
   if (m->mode == FIESTA_MODE_EXACT && m->X.key_base + m->n_ev >= FB_KEY_MASK) { set_error("more than 2^44 observations between two UpdateOccupancy calls"); return FIESTA_ERR_LIMIT; }
-  FbTouch t = {m->cnt, m->touch_flag, m->touch_list, m->touch_epoch, m->d_ctr, m->mode == FIESTA_MODE_EXACT ? m->X.tkey : nullptr, m->X.key_hi};
+  FbTouch t = {m->cnt, m->touch_flag, m->touch_list, m->touch_epoch, m->d_ctr, m->mode == FIESTA_MODE_EXACT ? m->X.tkey.get() : nullptr, m->X.key_hi};
   k_apply_events<<<(unsigned)((m->n_ev + 255) / 256), 256, 0, m->stream>>>(m->g, m->d_ev, m->n_ev, t, m->X.key_base);
   m->X.key_base += m->n_ev;
   m->st.kernel_launches++;
@@ -347,7 +344,7 @@ static int flush_events(fiesta_map *m) {
   return FIESTA_OK;
 }
 static inline int stage_event(fiesta_map *m, const int *v, int occ) {
-  if (m->n_ev == m->cap_ev) { int r = flush_events(m); if (r) return r; }
+  if (m->n_ev == m->h_ev.size()) { int r = flush_events(m); if (r) return r; }
   const long long ii = fb_ii(m->g, v[0], v[1], v[2]);
   m->pending_obs = true;
   m->h_ev[m->n_ev++] = (uint32_t)ii | ((uint32_t)occ << 31);
@@ -370,21 +367,9 @@ const char *fiesta_last_error(void) { return g_last_error.c_str(); }
 void fiesta_host_mirror_destroy(struct fiesta_host_mirror *p);
 void fiesta_destroy(fiesta_map *m) {
   if (!m) return;
-  cudaSetDevice(m->device);
+  cudaSetDevice(m->device);                                               // its buffers are freed on the device that holds them
   if (m->mirror) fiesta_host_mirror_destroy(m->mirror);                   // a mirror still attached goes with its map
   if (m->stream) cudaStreamSynchronize(m->stream);
-  void *dev[] = {m->cobs, m->cobs_b, m->stamp[0], m->stamp[1], m->occbits, m->occ, m->cnt, m->tile_flag, m->nb_flag, m->list[0], m->list[1],
-                 m->changed[0], m->changed[1], m->changed_bbox[0], m->changed_bbox[1], m->touch_flag, m->touch_list, m->ins, m->del, m->d_ctr, m->d_ev,
-                 m->d_xyz, m->ray_list, m->ray_len, m->ray_reach, m->ray_dirty, m->d_qin, m->d_qout};
-  for (void *p : dev) if (p) cudaFree(p);
-  if (m->mode == FIESTA_MODE_EXACT) fb_exact_free(&m->X);
-  if (m->d_dbg) cudaFree(m->d_dbg);
-  if (m->d_halo_changed) cudaFree(m->d_halo_changed);
-  { void *q[] = {m->d_img[0], m->d_img[1], m->d_dpts, m->d_dcloud, m->d_dflags, m->d_dsel, m->d_dcount, m->d_dtmp}; for (void *x : q) if (x) cudaFree(x); }
-  if (m->h_ctr) cudaFreeHost(m->h_ctr);
-  if (m->h_ev) cudaFreeHost(m->h_ev);
-  for (int i = 0; i < 4; ++i) if (m->ev[i]) cudaEventDestroy(m->ev[i]);
-  if (m->stream) cudaStreamDestroy(m->stream);
   delete m;
 }
 
@@ -400,9 +385,8 @@ int fiesta_create(const fiesta_config *cfg, fiesta_map **out) {
   CK(cudaGetDeviceProperties(&prop, cfg->device));
   if (prop.major != 10) { set_error("fiesta_create: device is not sm_100 (%s); this build only contains sm_100a code", prop.name); return FIESTA_ERR_NO_DEVICE; }
   CK(cudaSetDevice(cfg->device));
-  fiesta_map *m = new (std::nothrow) fiesta_map();
+  std::unique_ptr<fiesta_map> m(new (std::nothrow) fiesta_map());       // freed on every error return below
   if (!m) { set_error("out of host memory"); return FIESTA_ERR_INVALID; }
-  memset((void *)m, 0, sizeof(*m));
   m->device = cfg->device;
   m->mode = cfg->mode == FIESTA_MODE_FAST ? FIESTA_MODE_FAST : FIESTA_MODE_EXACT;
   if (const char *em = getenv("FIESTA_B200_MODE")) {                    // documented override (include/fiesta_b200.h)
@@ -421,13 +405,13 @@ int fiesta_create(const fiesta_config *cfg, fiesta_map **out) {
   }
   g.res = cfg->resolution; g.res_inv = 1 / cfg->resolution;
   if (gs[0] < 1 || gs[1] < 1 || gs[2] < 1 || gs[0] > FB_MAX_GX || gs[1] > FB_MAX_GY || gs[2] > FB_MAX_GZ) {
-    set_error("fiesta_create: grid exceeds the supported 2046 x 1024 x 1024 voxels"); delete m; return FIESTA_ERR_LIMIT;
+    set_error("fiesta_create: grid exceeds the supported 2046 x 1024 x 1024 voxels"); return FIESTA_ERR_LIMIT;
   }
   g.gx = gs[0]; g.gy = gs[1]; g.gz = gs[2]; g.pz = (g.gz + 3) & ~3;
   g.gyz = g.gy * g.gz;
   const long long total = (long long)g.gx * g.gyz;
   g.ptotal = (long long)g.gx * g.gy * g.pz;
-  if (total > 0x7fffffffLL || g.ptotal > (long long)FB_LIST_IDX_MASK) { set_error("fiesta_create: more than 2^30 voxels"); delete m; return FIESTA_ERR_LIMIT; }
+  if (total > 0x7fffffffLL || g.ptotal > (long long)FB_LIST_IDX_MASK) { set_error("fiesta_create: more than 2^30 voxels"); return FIESTA_ERR_LIMIT; }
   g.total = (int)total;
   g.tx = (g.gx + 7) / 8; g.ty = (g.gy + 7) / 8; g.tz = (g.gz + 7) / 8; g.ntiles = g.tx * g.ty * g.tz;
   for (int i = 0; i < 3; ++i) { g.min_vec[i] = g.last_min_vec[i] = 0; }   // SetOriginalRange, ESDFMap.cpp:819-822
@@ -435,50 +419,43 @@ int fiesta_create(const fiesta_config *cfg, fiesta_map **out) {
   set_box_flag(g);
   m->tile_x_lo = 0; m->tile_x_hi = g.tx;
 
-#define CKD(call)                                                                        \
-  do {                                                                                   \
-    cudaError_t e__ = (call);                                                            \
-    if (e__ != cudaSuccess) { set_error("%s failed: %s", #call, cudaGetErrorString(e__)); fiesta_destroy(m); return FIESTA_ERR_CUDA; } \
-  } while (0)
-  CKD(cudaStreamCreateWithFlags(&m->stream, cudaStreamNonBlocking));
-  for (int i = 0; i < 4; ++i) CKD(cudaEventCreate(&m->ev[i]));
+  CK(cudaStreamCreateWithFlags(&m->stream, cudaStreamNonBlocking));
+  for (int i = 0; i < 4; ++i) CK(cudaEventCreate(&m->ev[i]));
   const size_t P = (size_t)g.ptotal;
   const size_t nbits = (P + 31) / 32;
-  CKD(cudaMalloc((void **)&m->cobs, P * 4)); CKD(cudaMalloc((void **)&m->cobs_b, P * 4));
-  CKD(cudaMalloc((void **)&m->stamp[0], P * 4)); CKD(cudaMalloc((void **)&m->stamp[1], P * 4));
-  CKD(cudaMalloc((void **)&m->occbits, nbits * 4));
-  CKD(cudaMalloc((void **)&m->occ, P * 8)); CKD(cudaMalloc((void **)&m->cnt, P * 8));
-  CKD(cudaMalloc((void **)&m->touch_flag, (size_t)g.ntiles * 4)); CKD(cudaMalloc((void **)&m->touch_list, (size_t)g.ntiles * 4));
-  CKD(cudaMalloc((void **)&m->tile_flag, (size_t)g.ntiles * 4)); CKD(cudaMalloc((void **)&m->nb_flag, (size_t)g.ntiles * 4));
+  CK(m->cobs.alloc(P)); CK(m->cobs_b.alloc(P));
+  CK(m->stamp[0].alloc(P)); CK(m->stamp[1].alloc(P));
+  CK(m->occbits.alloc(nbits));
+  CK(m->occ.alloc(P)); CK(m->cnt.alloc(P));
+  CK(m->touch_flag.alloc(g.ntiles)); CK(m->touch_list.alloc(g.ntiles));
+  CK(m->tile_flag.alloc(g.ntiles)); CK(m->nb_flag.alloc(g.ntiles));
   for (int k = 0; k < 2; ++k) {
-    CKD(cudaMalloc((void **)&m->list[k], (size_t)g.ntiles * 4));
-    CKD(cudaMalloc((void **)&m->changed[k], (size_t)g.ntiles * 4));
-    CKD(cudaMalloc((void **)&m->changed_bbox[k], (size_t)g.ntiles * 4));
+    CK(m->list[k].alloc(g.ntiles));
+    CK(m->changed[k].alloc(g.ntiles));
+    CK(m->changed_bbox[k].alloc(g.ntiles));
   }
-  CKD(cudaMalloc((void **)&m->d_ctr, sizeof(FbCounters)));
-  CKD(cudaMallocHost((void **)&m->h_ctr, sizeof(FbCounters)));
-  m->cap_ev = 1u << 22;
-  CKD(cudaMallocHost((void **)&m->h_ev, m->cap_ev * 4)); CKD(cudaMalloc((void **)&m->d_ev, m->cap_ev * 4));
-  CKD(cudaMemsetAsync(m->cobs, 0, P * 4, m->stream)); CKD(cudaMemsetAsync(m->cobs_b, 0, P * 4, m->stream));
-  CKD(cudaMemsetAsync(m->stamp[0], 0, P * 4, m->stream)); CKD(cudaMemsetAsync(m->stamp[1], 0, P * 4, m->stream));
-  CKD(cudaMemsetAsync(m->occbits, 0, nbits * 4, m->stream));
-  CKD(cudaMemsetAsync(m->occ, 0, P * 8, m->stream)); CKD(cudaMemsetAsync(m->cnt, 0, P * 8, m->stream));
-  CKD(cudaMemsetAsync(m->tile_flag, 0, (size_t)g.ntiles * 4, m->stream)); CKD(cudaMemsetAsync(m->nb_flag, 0, (size_t)g.ntiles * 4, m->stream));
-  CKD(cudaMemsetAsync(m->touch_flag, 0, (size_t)g.ntiles * 4, m->stream));
+  CK(m->d_ctr.alloc(1));
+  CK(m->h_ctr.alloc(1));
+  CK(m->h_ev.alloc(1u << 22)); CK(m->d_ev.alloc(1u << 22));
+  CK(cudaMemsetAsync(m->cobs, 0, P * 4, m->stream)); CK(cudaMemsetAsync(m->cobs_b, 0, P * 4, m->stream));
+  CK(cudaMemsetAsync(m->stamp[0], 0, P * 4, m->stream)); CK(cudaMemsetAsync(m->stamp[1], 0, P * 4, m->stream));
+  CK(cudaMemsetAsync(m->occbits, 0, nbits * 4, m->stream));
+  CK(cudaMemsetAsync(m->occ, 0, P * 8, m->stream)); CK(cudaMemsetAsync(m->cnt, 0, P * 8, m->stream));
+  CK(cudaMemsetAsync(m->tile_flag, 0, (size_t)g.ntiles * 4, m->stream)); CK(cudaMemsetAsync(m->nb_flag, 0, (size_t)g.ntiles * 4, m->stream));
+  CK(cudaMemsetAsync(m->touch_flag, 0, (size_t)g.ntiles * 4, m->stream));
   m->touch_epoch = 1;
   memset(m->h_ctr, 0, sizeof(FbCounters));
   m->h_ctr->gen_stamp = 1;
-  CKD(cudaMemcpyAsync(m->d_ctr, m->h_ctr, sizeof(FbCounters), cudaMemcpyHostToDevice, m->stream));
+  CK(cudaMemcpyAsync(m->d_ctr, m->h_ctr, sizeof(FbCounters), cudaMemcpyHostToDevice, m->stream));
   m->frame_tag = 0; m->owner_tag = 0;
   char err[256];
-  if (fb_esdf_make_tensor_map(&m->tmap, g, m->cobs, err, sizeof(err)) != cudaSuccess) { set_error("%s", err); fiesta_destroy(m); return FIESTA_ERR_CUDA; }
+  if (fb_esdf_make_tensor_map(&m->tmap, g, m->cobs, err, sizeof(err)) != cudaSuccess) { set_error("%s", err); return FIESTA_ERR_CUDA; }
   m->wf_blocks = fb_esdf_wavefront_blocks(m->device);
   m->rr_blocks = fb_ray_resolve_blocks(m->device);
-  if (m->wf_blocks <= 0 || m->rr_blocks <= 0) { set_error("cooperative kernels do not fit on this device"); fiesta_destroy(m); return FIESTA_ERR_CUDA; }
-  if (m->mode == FIESTA_MODE_EXACT && fb_exact_init(&m->X, g, m->device, m->stream) != cudaSuccess) { set_error("exact mode init: %s", m->X.err); fiesta_destroy(m); return FIESTA_ERR_CUDA; }
-  CKD(cudaStreamSynchronize(m->stream));
-#undef CKD
-  *out = m;
+  if (m->wf_blocks <= 0 || m->rr_blocks <= 0) { set_error("cooperative kernels do not fit on this device"); return FIESTA_ERR_CUDA; }
+  if (m->mode == FIESTA_MODE_EXACT && fb_exact_init(&m->X, g, m->device, m->stream) != cudaSuccess) { set_error("exact mode init: %s", m->X.err); return FIESTA_ERR_CUDA; }
+  CK(cudaStreamSynchronize(m->stream));
+  *out = m.release();
   return FIESTA_OK;
 }
 
@@ -614,25 +591,18 @@ int fiesta_raycast_frame_device(fiesta_map *m, const float *d_xyz, int64_t n, co
   a.frame_tag = ++m->frame_tag;
   a.owner_tag = ++m->owner_tag;
   int r;
-  size_t need_rays = (size_t)n;
-  if (need_rays > m->cap_rays) {
-    size_t c1 = m->cap_rays, c2 = m->cap_rays, c4 = m->cap_rays;
-    if ((r = ensure(&m->ray_len, &c1, need_rays, false, m->stream))) return r;
-    if ((r = ensure(&m->ray_reach, &c2, need_rays, false, m->stream))) return r;
-    if ((r = ensure(&m->ray_dirty, &c4, need_rays, false, m->stream))) return r;
-    m->cap_rays = c1;
-    if (c2 < m->cap_rays) m->cap_rays = c2;
-    if (c4 < m->cap_rays) m->cap_rays = c4;
-  }
-  if ((r = ensure(&m->ray_list, &m->cap_ray_list, (size_t)a.cap * (size_t)n, false, m->stream))) return r;
+  CK(m->ray_len.reserve((size_t)n, m->stream, false));
+  CK(m->ray_reach.reserve((size_t)n, m->stream, false));
+  CK(m->ray_dirty.reserve((size_t)n, m->stream, false));
+  CK(m->ray_list.reserve((size_t)a.cap * (size_t)n, m->stream, false));
   a.cnt = m->cnt; a.stamp[0] = m->stamp[0]; a.stamp[1] = m->stamp[1];
   a.touch_flag = m->touch_flag; a.touch_list = m->touch_list; a.touch_epoch = m->touch_epoch;
-  a.tkey = m->mode == FIESTA_MODE_EXACT ? m->X.tkey : nullptr; a.key_hi = m->X.key_hi; a.key_base = m->X.key_base;
+  a.tkey = m->mode == FIESTA_MODE_EXACT ? m->X.tkey.get() : nullptr; a.key_hi = m->X.key_hi; a.key_base = m->X.key_base;
   m->X.key_base += 1ull << 30;                                            // (point index << 11) + position along the ray < 2^30
   a.ray_list = m->ray_list; a.ray_len = m->ray_len; a.ray_reach = m->ray_reach; a.ray_dirty = m->ray_dirty; a.ctr = m->d_ctr;
   static const bool dbg_ray = getenv("FIESTA_DEBUG_RAY") != nullptr;
   a.dbg = nullptr;
-  if (dbg_ray) { if (!m->d_dbg) CK(cudaMalloc((void **)&m->d_dbg, 2048 * 8)); CK(cudaMemsetAsync(m->d_dbg, 0, 2048 * 8, m->stream)); a.dbg = m->d_dbg; }
+  if (dbg_ray) { if (!m->d_dbg) CK(m->d_dbg.alloc(2048)); CK(cudaMemsetAsync(m->d_dbg, 0, 2048 * 8, m->stream)); a.dbg = m->d_dbg; }
   CK(cudaEventRecord(m->ev[0], m->stream));
   k_reset_ray_ctr<<<1, 1, 0, m->stream>>>(m->d_ctr);
   int launches = 1;
@@ -658,8 +628,7 @@ int fiesta_raycast_frame_device(fiesta_map *m, const float *d_xyz, int64_t n, co
 int fiesta_raycast_frame(fiesta_map *m, const float *xyz, int64_t n, const double T[16], const fiesta_raycast_params *p) {
   if (!m || n < 0 || (n > 0 && !xyz)) { set_error("fiesta_raycast_frame: bad argument"); return FIESTA_ERR_INVALID; }
   CK(cudaSetDevice(m->device));
-  int r;
-  if ((r = ensure(&m->d_xyz, &m->cap_xyz, (size_t)n * 3, false, m->stream))) return r;
+  CK(m->d_xyz.reserve((size_t)n * 3, m->stream, false));
   if (n) CK(cudaMemcpyAsync(m->d_xyz, xyz, (size_t)n * 3 * sizeof(float), cudaMemcpyHostToDevice, m->stream));
   return fiesta_raycast_frame_device(m, m->d_xyz, n, T, p);
 }
@@ -669,14 +638,12 @@ int fiesta_depth_frame(fiesta_map *m, const uint16_t *depth, int rows, int cols,
   if (!m || !depth || !dp || !T || !rp || rows <= 0 || cols <= 0) { set_error("fiesta_depth_frame: bad argument"); return FIESTA_ERR_INVALID; }
   CK(cudaSetDevice(m->device));
   const size_t N = (size_t)rows * cols;
-  if (N > m->cap_img) {
-    void *q[] = {m->d_img[0], m->d_img[1], m->d_dpts, m->d_dcloud, m->d_dflags, m->d_dsel};
-    for (void *x : q) if (x) cudaFree(x);
-    m->d_img[0] = m->d_img[1] = nullptr; m->d_dpts = m->d_dcloud = nullptr; m->d_dflags = nullptr; m->d_dsel = nullptr; m->cap_img = 0;
-    CK(cudaMalloc((void **)&m->d_img[0], N * 2)); CK(cudaMalloc((void **)&m->d_img[1], N * 2));
-    CK(cudaMalloc((void **)&m->d_dpts, N * 12)); CK(cudaMalloc((void **)&m->d_dcloud, N * 12));
-    CK(cudaMalloc((void **)&m->d_dflags, N)); CK(cudaMalloc((void **)&m->d_dsel, N * 4));
-    if (!m->d_dcount) CK(cudaMalloc((void **)&m->d_dcount, 16));
+  if (N > m->cap_img) {                                                   // exact sizes: a larger image restarts the depth filter
+    m->cap_img = 0;
+    CK(m->d_img[0].alloc(N)); CK(m->d_img[1].alloc(N));
+    CK(m->d_dpts.alloc(N * 3)); CK(m->d_dcloud.alloc(N * 3));
+    CK(m->d_dflags.alloc(N)); CK(m->d_dsel.alloc(N));
+    if (!m->d_dcount) CK(m->d_dcount.alloc(4));
     m->cap_img = N; m->image_cnt = 0;
   }
   ++m->image_cnt;                                                          // Fiesta.h:321-323: img_[image_cnt_ & 1] is the current image
@@ -692,7 +659,7 @@ int fiesta_depth_frame(fiesta_map *m, const uint16_t *depth, int rows, int cols,
   FbDepthRel rel;
   for (int k = 0; k < 16; ++k) rel.m[k] = (dp->use_depth_filter && m_rel) ? m_rel[k] : (k % 5 == 0 ? 1.0 : 0.0);
   CK(fb_depth_to_cloud(cur, last, rows, cols, *dp, dp->use_depth_filter ? 1 : 0, rel, m->d_dpts, m->d_dflags, m->d_dsel, m->d_dcloud, m->d_dcount,
-                       &m->d_dtmp, &m->d_dtmp_bytes, &n, m->stream));
+                       m->d_dtmp, &n, m->stream));
   m->st.kernel_launches += 3;
   m->last_cloud_n = n;
   if (n_points) *n_points = n;
@@ -731,14 +698,14 @@ int fiesta_update_occupancy(fiesta_map *m, int global_map) {
       cudaMemsetAsync(X.d_count, 0, 8, m->stream);
       const unsigned blocks = n < 148u * 16u ? n : 148u * 16u;
       // crossings are staged (voxel, first-observation time) in arrays that are scratch between two k_x_relax launches
-      unsigned long long *ikey = reinterpret_cast<unsigned long long *>(X.SUM), *dkey = ikey + m->g.ptotal;
+      unsigned long long *ikey = reinterpret_cast<unsigned long long *>(X.SUM.get()), *dkey = ikey + m->g.ptotal;
       k_integrate<true><<<blocks, 128, 0, m->stream>>>(m->g, m->touch_list, n, m->cnt, m->occ, m->cobs, m->occbits, X.touched, X.emask, X.d_count, X.d_count + 1,
                                                        m->d_ctr, X.tkey, ikey, dkey, global_map, m->l_hit, m->l_miss, m->l_min, m->l_max, m->l_occ);
       k_reset_queues<<<1, 1, 0, m->stream>>>(m->d_ctr, 1, 0);
       m->touch_epoch++;
       m->st.kernel_launches += 3;
       int launches = 0;
-      if (fb_exact_queue_crossings(&X, ikey, X.touched, dkey, X.emask, &m->ins, &m->cap_ins, &m->n_ins, &m->del, &m->cap_del, &m->n_del, m->stream, &launches) != cudaSuccess) {
+      if (fb_exact_queue_crossings(&X, ikey, X.touched, dkey, X.emask, m->ins, &m->n_ins, m->del, &m->n_del, m->stream, &launches) != cudaSuccess) {
         set_error("exact UpdateOccupancy: %s", X.err); return -FIESTA_ERR_CUDA;
       }
       m->st.kernel_launches += launches;
@@ -752,8 +719,9 @@ int fiesta_update_occupancy(fiesta_map *m, int global_map) {
     return (m->n_ins > 0 || m->n_del > 0) ? 1 : 0;
   }
   if (n) {
-    if ((r = ensure(&m->ins, &m->cap_ins, (size_t)m->n_ins + (size_t)n * 512, true, m->stream))) return -r;
-    if ((r = ensure(&m->del, &m->cap_del, (size_t)m->n_del + (size_t)n * 512, true, m->stream))) return -r;
+    cudaError_t e = m->ins.reserve((size_t)m->n_ins + (size_t)n * 512, m->stream, true);   // pushes not yet consumed by UpdateESDF stay
+    if (e == cudaSuccess) e = m->del.reserve((size_t)m->n_del + (size_t)n * 512, m->stream, true);
+    if (e != cudaSuccess) { set_error("UpdateOccupancy: growing the queues failed: %s", cudaGetErrorString(e)); return -FIESTA_ERR_CUDA; }
     k_reset_touched<<<1, 1, 0, m->stream>>>(m->d_ctr);
     const unsigned blocks = n < 148u * 16u ? n : 148u * 16u;
     k_integrate<false><<<blocks, 128, 0, m->stream>>>(m->g, m->touch_list, n, m->cnt, m->occ, m->cobs, m->occbits, m->ins, m->del, &m->d_ctr->n_ins, &m->d_ctr->n_del,
@@ -805,7 +773,7 @@ int fiesta_update_esdf(fiesta_map *m) {
   a.tile_x_lo = m->tile_x_lo; a.tile_x_hi = m->tile_x_hi;
   a.dbg = nullptr;
   static const bool dbg_wf = getenv("FIESTA_DEBUG_WF") != nullptr;
-  if (dbg_wf) { if (!m->d_dbg) CK(cudaMalloc((void **)&m->d_dbg, 2048 * 8)); CK(cudaMemsetAsync(m->d_dbg, 0, 2048 * 8, m->stream)); a.dbg = m->d_dbg; }
+  if (dbg_wf) { if (!m->d_dbg) CK(m->d_dbg.alloc(2048)); CK(cudaMemsetAsync(m->d_dbg, 0, 2048 * 8, m->stream)); a.dbg = m->d_dbg; }
   CK(cudaEventRecord(m->ev[0], m->stream));
   k_reset_esdf_ctr<<<1, 1, 0, m->stream>>>(m->d_ctr);
   m->st.kernel_launches++;
@@ -870,14 +838,8 @@ int fiesta_set_original_range(fiesta_map *m) {
 static int run_query(fiesta_map *m, const double *pos, int64_t n, int mode, double *out, double *grad) {
   if (n <= 0) return FIESTA_OK;
   CK(cudaSetDevice(m->device));
-  int r;
-  size_t c1 = m->cap_q, c2 = m->cap_q;
-  if ((size_t)n * 3 > m->cap_q) {
-    if ((r = ensure(&m->d_qin, &c1, (size_t)n * 3, false, m->stream))) return r;
-    if ((r = ensure(&m->d_qout, &c2, (size_t)n * 4, false, m->stream))) return r;   // [dist n][grad 3n]
-    m->cap_q = (c1 < c2 ? c1 : c2) * 3 / 4;
-    if (m->cap_q < (size_t)n * 3) m->cap_q = (size_t)n * 3;
-  }
+  CK(m->d_qin.reserve((size_t)n * 3, m->stream, false));
+  CK(m->d_qout.reserve((size_t)n * 4, m->stream, false));                 // [dist n][grad 3n]
   CK(cudaMemcpyAsync(m->d_qin, pos, (size_t)n * 3 * sizeof(double), cudaMemcpyHostToDevice, m->stream));
   k_query<<<(unsigned)((n + 127) / 128), 128, 0, m->stream>>>(m->g, m->cobs, m->occ, m->l_occ, m->d_qin, n, mode, m->d_qout, m->d_qout + n);
   m->st.kernel_launches++;
@@ -940,21 +902,19 @@ int fiesta_get_dist_grad_trilinear_batch(fiesta_map *m, const double *pos, int64
 struct fiesta_query_plan {
   fiesta_map *m;
   int64_t n;
-  double *h_pos, *h_out;        // pinned: [3n] positions; [n] distances followed by [3n] gradients
-  double *d_pos, *d_out;
+  FbPinned<double> h_pos, h_out;  // [3n] positions; [n] distances followed by [3n] gradients.  The graph captured these
+  FbDev<double> d_pos, d_out;     // addresses (and the map's cobs / occ): none of them is ever reallocated
   cudaGraph_t graph;
   cudaGraphExec_t exec;
+  ~fiesta_query_plan() {
+    if (exec) cudaGraphExecDestroy(exec);
+    if (graph) cudaGraphDestroy(graph);
+  }
 };
 void fiesta_query_plan_destroy(fiesta_query_plan *p) {
   if (!p) return;
   cudaSetDevice(p->m->device);
   cudaStreamSynchronize(p->m->stream);
-  if (p->exec) cudaGraphExecDestroy(p->exec);
-  if (p->graph) cudaGraphDestroy(p->graph);
-  if (p->h_pos) cudaFreeHost(p->h_pos);
-  if (p->h_out) cudaFreeHost(p->h_out);
-  if (p->d_pos) cudaFree(p->d_pos);
-  if (p->d_out) cudaFree(p->d_out);
   delete p;
 }
 int fiesta_query_plan_create(fiesta_map *m, int64_t n, fiesta_query_plan **out) {
@@ -962,28 +922,25 @@ int fiesta_query_plan_create(fiesta_map *m, int64_t n, fiesta_query_plan **out) 
   if (!m->params_set) { set_error("fiesta_query_plan_create: call SetParameters first (the occupancy threshold is captured)"); return FIESTA_ERR_INVALID; }
   *out = nullptr;
   CK(cudaSetDevice(m->device));
-  fiesta_query_plan *p = new (std::nothrow) fiesta_query_plan();
+  std::unique_ptr<fiesta_query_plan> p(new (std::nothrow) fiesta_query_plan());
   if (!p) return FIESTA_ERR_INVALID;
-  memset((void *)p, 0, sizeof(*p));
   p->m = m; p->n = n;
-#define CKP(call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) { set_error("%s failed: %s", #call, cudaGetErrorString(e__)); fiesta_query_plan_destroy(p); return FIESTA_ERR_CUDA; } } while (0)
-  CKP(cudaMallocHost((void **)&p->h_pos, (size_t)n * 3 * sizeof(double)));
-  CKP(cudaMallocHost((void **)&p->h_out, (size_t)n * 4 * sizeof(double)));
-  CKP(cudaMalloc((void **)&p->d_pos, (size_t)n * 3 * sizeof(double)));
-  CKP(cudaMalloc((void **)&p->d_out, (size_t)n * 4 * sizeof(double)));
-  CKP(cudaStreamSynchronize(m->stream));
-  CKP(cudaStreamBeginCapture(m->stream, cudaStreamCaptureModeThreadLocal));
+  CK(p->h_pos.alloc((size_t)n * 3));
+  CK(p->h_out.alloc((size_t)n * 4));
+  CK(p->d_pos.alloc((size_t)n * 3));
+  CK(p->d_out.alloc((size_t)n * 4));
+  CK(cudaStreamSynchronize(m->stream));
+  CK(cudaStreamBeginCapture(m->stream, cudaStreamCaptureModeThreadLocal));
   cudaMemcpyAsync(p->d_pos, p->h_pos, (size_t)n * 3 * sizeof(double), cudaMemcpyHostToDevice, m->stream);
   k_query<<<(unsigned)((n + 127) / 128), 128, 0, m->stream>>>(m->g, m->cobs, m->occ, m->l_occ, p->d_pos, n, 1, p->d_out, p->d_out + n);
   cudaMemcpyAsync(p->h_out, p->d_out, (size_t)n * 4 * sizeof(double), cudaMemcpyDeviceToHost, m->stream);
-  CKP(cudaStreamEndCapture(m->stream, &p->graph));
-  CKP(cudaGraphInstantiate(&p->exec, p->graph, 0));
-#undef CKP
-  *out = p;
+  CK(cudaStreamEndCapture(m->stream, &p->graph));
+  CK(cudaGraphInstantiate(&p->exec, p->graph, 0));
+  *out = p.release();
   return FIESTA_OK;
 }
-double *fiesta_query_plan_positions(fiesta_query_plan *p) { return p ? p->h_pos : nullptr; }
-const double *fiesta_query_plan_distances(const fiesta_query_plan *p) { return p ? p->h_out : nullptr; }
+double *fiesta_query_plan_positions(fiesta_query_plan *p) { return p ? p->h_pos.get() : nullptr; }
+const double *fiesta_query_plan_distances(const fiesta_query_plan *p) { return p ? p->h_out.get() : nullptr; }
 const double *fiesta_query_plan_gradients(const fiesta_query_plan *p) { return p ? p->h_out + p->n : nullptr; }
 int fiesta_query_plan_run(fiesta_query_plan *p) {
   if (!p) return FIESTA_ERR_INVALID;
@@ -1001,11 +958,12 @@ int fiesta_query_plan_run(fiesta_query_plan *p) {
 // word, so a reader racing a refresh sees the old or the new record of a voxel, never a torn one.
 struct fiesta_host_mirror {
   fiesta_map *m;
-  uint32_t *h_rec;                // pinned [ptotal]
-  uint32_t *d_shadow;             // device [ptotal]: the records the host holds
-  uint2 *d_chg, *h_chg;           // change list, device + pinned
-  size_t cap_chg;
-  unsigned *d_n, *h_n;
+  FbPinned<uint32_t> h_rec;       // [ptotal]; fiesta_host_mirror_records hands this address out: never reallocated
+  FbDev<uint32_t> d_shadow;       // [ptotal]: the records the host holds
+  FbDev<uint2> d_chg;             // change list, device + pinned
+  FbPinned<uint2> h_chg;
+  FbDev<unsigned> d_n;
+  FbPinned<unsigned> h_n;
   int64_t last_changed, last_scanned, refreshes, full_copies;
 };
 __global__ void k_mirror_diff(FbGeom g, const uint32_t *cobs, uint32_t *shadow, int lx, int ly, int lz, int ex, int ey, int ez, uint2 *chg,
@@ -1026,12 +984,6 @@ void fiesta_host_mirror_destroy(fiesta_host_mirror *p) {
   cudaSetDevice(p->m->device);
   cudaStreamSynchronize(p->m->stream);
   if (p->m->mirror == p) p->m->mirror = nullptr;
-  if (p->h_rec) cudaFreeHost(p->h_rec);
-  if (p->h_chg) cudaFreeHost(p->h_chg);
-  if (p->h_n) cudaFreeHost(p->h_n);
-  if (p->d_shadow) cudaFree(p->d_shadow);
-  if (p->d_chg) cudaFree(p->d_chg);
-  if (p->d_n) cudaFree(p->d_n);
   delete p;
 }
 static int mirror_full_copy(fiesta_host_mirror *p) {
@@ -1048,28 +1000,25 @@ int fiesta_host_mirror_create(fiesta_map *m, fiesta_host_mirror **out) {
   *out = nullptr;
   if (m->mirror) { set_error("fiesta_host_mirror_create: this map already has a host mirror"); return FIESTA_ERR_INVALID; }
   CK(cudaSetDevice(m->device));
-  fiesta_host_mirror *p = new (std::nothrow) fiesta_host_mirror();
+  std::unique_ptr<fiesta_host_mirror> p(new (std::nothrow) fiesta_host_mirror());
   if (!p) return FIESTA_ERR_INVALID;
-  memset((void *)p, 0, sizeof(*p));
   p->m = m;
   const size_t P = (size_t)m->g.ptotal;
-  p->cap_chg = P / 32 > (1u << 20) ? P / 32 : (1u << 20);
-  if (p->cap_chg > P) p->cap_chg = P;
-  if (const char *e = getenv("FIESTA_MIRROR_CAP")) { const long v = atol(e); if (v > 0 && (size_t)v < p->cap_chg) p->cap_chg = (size_t)v; }   // tests: force the bulk-copy path
-#define CKP(call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) { set_error("%s failed: %s", #call, cudaGetErrorString(e__)); fiesta_host_mirror_destroy(p); return FIESTA_ERR_CUDA; } } while (0)
-  CKP(cudaMallocHost((void **)&p->h_rec, P * 4));
-  CKP(cudaMallocHost((void **)&p->h_chg, p->cap_chg * sizeof(uint2)));
-  CKP(cudaMallocHost((void **)&p->h_n, 4));
-  CKP(cudaMalloc((void **)&p->d_shadow, P * 4));
-  CKP(cudaMalloc((void **)&p->d_chg, p->cap_chg * sizeof(uint2)));
-  CKP(cudaMalloc((void **)&p->d_n, 4));
-#undef CKP
+  size_t cap_chg = P / 32 > (1u << 20) ? P / 32 : (1u << 20);
+  if (cap_chg > P) cap_chg = P;
+  if (const char *e = getenv("FIESTA_MIRROR_CAP")) { const long v = atol(e); if (v > 0 && (size_t)v < cap_chg) cap_chg = (size_t)v; }   // tests: force the bulk-copy path
+  CK(p->h_rec.alloc(P));
+  CK(p->h_chg.alloc(cap_chg));
+  CK(p->h_n.alloc(1));
+  CK(p->d_shadow.alloc(P));
+  CK(p->d_chg.alloc(cap_chg));
+  CK(p->d_n.alloc(1));
   int r = flush_events(m);
-  if (!r) r = mirror_full_copy(p);
-  if (r) { fiesta_host_mirror_destroy(p); return r; }
+  if (!r) r = mirror_full_copy(p.get());
+  if (r) return r;
   p->full_copies = 0;
-  m->mirror = p;                                                          // the dirty box is kept: the first refresh rescans it
-  *out = p;
+  m->mirror = p.release();                                                // the dirty box is kept: the first refresh rescans it
+  *out = m->mirror;
   return FIESTA_OK;
 }
 int fiesta_host_mirror_refresh(fiesta_host_mirror *p, int64_t *n_changed) {
@@ -1097,7 +1046,7 @@ int fiesta_host_mirror_refresh(fiesta_host_mirror *p, int64_t *n_changed) {
   CK(cudaMemsetAsync(p->d_n, 0, 4, m->stream));
   const long long want = (vol + 255) / 256;
   const unsigned blocks = (unsigned)(want < 148ll * 16 ? want : 148ll * 16);
-  k_mirror_diff<<<blocks, 256, 0, m->stream>>>(g, m->cobs, p->d_shadow, lo[0], lo[1], lo[2], ex[0], ex[1], ex[2], p->d_chg, (unsigned)p->cap_chg, p->d_n);
+  k_mirror_diff<<<blocks, 256, 0, m->stream>>>(g, m->cobs, p->d_shadow, lo[0], lo[1], lo[2], ex[0], ex[1], ex[2], p->d_chg, (unsigned)p->d_chg.size(), p->d_n);
   m->st.kernel_launches++;
   CK(cudaGetLastError());
   CK(cudaMemcpyAsync(p->h_n, p->d_n, 4, cudaMemcpyDeviceToHost, m->stream));
@@ -1106,7 +1055,7 @@ int fiesta_host_mirror_refresh(fiesta_host_mirror *p, int64_t *n_changed) {
   p->last_changed = (int64_t)n;
   if (n_changed) *n_changed = (int64_t)n;
   if (n == 0) return FIESTA_OK;
-  if (n > p->cap_chg) return mirror_full_copy(p);                         // the shadow is already current; one bulk copy brings the host up
+  if (n > p->d_chg.size()) return mirror_full_copy(p);                    // the shadow is already current; one bulk copy brings the host up
   CK(cudaMemcpyAsync(p->h_chg, p->d_chg, n * sizeof(uint2), cudaMemcpyDeviceToHost, m->stream));
   CK(cudaStreamSynchronize(m->stream));
   for (size_t i = 0; i < n; ++i) {
@@ -1135,7 +1084,7 @@ int fiesta_host_mirror_get_dist_grad_trilinear_batch(const fiesta_host_mirror *p
   for (int64_t i = 0; i < n; ++i) out[i] = fb_query_trilinear(p->m->g, p->h_rec, pos + 3 * i, grad + 3 * i);
   return FIESTA_OK;
 }
-const uint32_t *fiesta_host_mirror_records(const fiesta_host_mirror *p) { return p ? p->h_rec : nullptr; }
+const uint32_t *fiesta_host_mirror_records(const fiesta_host_mirror *p) { return p ? p->h_rec.get() : nullptr; }
 int fiesta_host_mirror_stats(const fiesta_host_mirror *p, int64_t out[4]) {
   if (!p || !out) return FIESTA_ERR_INVALID;
   out[0] = p->last_changed; out[1] = p->last_scanned; out[2] = p->refreshes; out[3] = p->full_copies;
@@ -1146,12 +1095,12 @@ int fiesta_host_mirror_stats(const fiesta_host_mirror *p, int64_t out[4]) {
 static int run_export(fiesta_map *m, double *dist, int *cobs3, double *occ, int *hit, int *tot) {
   CK(cudaSetDevice(m->device));
   const size_t G = (size_t)m->g.total;
-  double *dd = nullptr, *dof = nullptr; int *dc = nullptr, *dh = nullptr, *dt = nullptr;
+  FbDev<double> dd, dof; FbDev<int> dc, dh, dt;
   cudaError_t e = cudaSuccess;
-  if (dist) e = cudaMalloc((void **)&dd, G * 8);
-  if (!e && occ) e = cudaMalloc((void **)&dof, G * 8);
-  if (!e && cobs3) e = cudaMalloc((void **)&dc, G * 12);
-  if (!e && hit) { e = cudaMalloc((void **)&dh, G * 4); if (!e) e = cudaMalloc((void **)&dt, G * 4); }
+  if (dist) e = dd.alloc(G);
+  if (!e && occ) e = dof.alloc(G);
+  if (!e && cobs3) e = dc.alloc(G * 3);
+  if (!e && hit) { e = dh.alloc(G); if (!e) e = dt.alloc(G); }
   if (!e) {
     k_export<<<(unsigned)((G + 255) / 256), 256, 0, m->stream>>>(m->g, m->cobs, m->occ, m->cnt, dd, dc, dof, dh, dt);
     m->st.kernel_launches++;
@@ -1162,7 +1111,6 @@ static int run_export(fiesta_map *m, double *dist, int *cobs3, double *occ, int 
   if (!e && cobs3) e = cudaMemcpyAsync(cobs3, dc, G * 12, cudaMemcpyDeviceToHost, m->stream);
   if (!e && hit) { e = cudaMemcpyAsync(hit, dh, G * 4, cudaMemcpyDeviceToHost, m->stream); if (!e) e = cudaMemcpyAsync(tot, dt, G * 4, cudaMemcpyDeviceToHost, m->stream); }
   if (!e) e = cudaStreamSynchronize(m->stream);
-  cudaFree(dd); cudaFree(dof); cudaFree(dc); cudaFree(dh); cudaFree(dt);
   if (e != cudaSuccess) { set_error("export failed: %s", cudaGetErrorString(e)); return FIESTA_ERR_CUDA; }
   return FIESTA_OK;
 }
@@ -1193,7 +1141,7 @@ int fiesta_set_shard(fiesta_map *m, int rank, int world, fiesta_shard_info *out)
   m->shard_rank = rank; m->shard_world = world;
   m->tile_x_lo = (int)((long long)m->g.tx * rank / world);
   m->tile_x_hi = (int)((long long)m->g.tx * (rank + 1) / world);
-  if (!m->d_halo_changed) CK(cudaMalloc((void **)&m->d_halo_changed, 16));
+  if (!m->d_halo_changed) CK(m->d_halo_changed.alloc(4));
   if (out) {
     out->rank = rank; out->world = world;
     out->x_begin = m->tile_x_lo * 8; out->x_end = m->tile_x_hi * 8 < m->g.gx ? m->tile_x_hi * 8 : m->g.gx;

@@ -68,34 +68,32 @@ __global__ void k_vis_slice_points(FbGeom g, const uint32_t *cobs, const uint32_
 }
 
 static cudaError_t vis_select(const uint8_t *flags, size_t n, uint32_t *sel, unsigned *count, cudaStream_t s) {
-  unsigned *d_cnt = nullptr; void *tmp = nullptr; size_t bytes = 0;
-  cudaError_t e = cudaMalloc((void **)&d_cnt, 4);
+  FbDev<unsigned> d_cnt; FbDev<uint8_t> tmp; size_t bytes = 0;
+  cudaError_t e = d_cnt.alloc(1);
   if (e) return e;
   thrust::counting_iterator<uint32_t> it(0);
-  e = cub::DeviceSelect::Flagged(nullptr, bytes, it, flags, sel, d_cnt, (int)n, s);
-  if (!e) e = cudaMalloc(&tmp, bytes ? bytes : 16);
-  if (!e) e = cub::DeviceSelect::Flagged(tmp, bytes, it, flags, sel, d_cnt, (int)n, s);
+  e = cub::DeviceSelect::Flagged(nullptr, bytes, it, flags, sel, d_cnt.get(), (int)n, s);
+  if (!e) e = tmp.alloc(bytes ? bytes : 16);
+  if (!e) e = cub::DeviceSelect::Flagged(tmp.get(), bytes, it, flags, sel, d_cnt.get(), (int)n, s);
   if (!e) e = cudaMemcpyAsync(count, d_cnt, 4, cudaMemcpyDeviceToHost, s);
   if (!e) e = cudaStreamSynchronize(s);
-  cudaFree(tmp); cudaFree(d_cnt);
   return e;
 }
 
 cudaError_t fb_vis_point_cloud(const FbGeom &g, const double *occ, double l_occ, int zlo, int zhi, float *h_out, long long cap, long long *count, cudaStream_t s) {
   const size_t G = (size_t)g.total;
-  uint8_t *flags = nullptr; uint32_t *sel = nullptr; float *pts = nullptr;
-  cudaError_t e = cudaMalloc((void **)&flags, G);
-  if (!e) e = cudaMalloc((void **)&sel, G * 4);
+  FbDev<uint8_t> flags; FbDev<uint32_t> sel; FbDev<float> pts;
+  cudaError_t e = flags.alloc(G);
+  if (!e) e = sel.alloc(G);
   unsigned n = 0;
   if (!e) { k_vis_occ_flags<<<(unsigned)((G + 255) / 256), 256, 0, s>>>(g, occ, l_occ, zlo, zhi, flags); e = vis_select(flags, G, sel, &n, s); }
   *count = n;
   const unsigned m = (long long)n < cap ? n : (unsigned)(cap < 0 ? 0 : cap);
   if (!e && m) {
-    e = cudaMalloc((void **)&pts, (size_t)m * 12);
+    e = pts.alloc((size_t)m * 3);
     if (!e) { k_vis_occ_points<<<(m + 255) / 256, 256, 0, s>>>(g, sel, m, pts); e = cudaMemcpyAsync(h_out, pts, (size_t)m * 12, cudaMemcpyDeviceToHost, s); }
     if (!e) e = cudaStreamSynchronize(s);
   }
-  cudaFree(flags); cudaFree(sel); cudaFree(pts);
   return e;
 }
 
@@ -103,16 +101,16 @@ cudaError_t fb_vis_slice(const FbGeom &g, const uint32_t *cobs, int slice, doubl
   *count = 0;
   if (slice < 0 || slice >= g.gz) return cudaSuccess;
   const size_t G = (size_t)g.gx * g.gy;
-  uint8_t *flags = nullptr; uint32_t *sel = nullptr; double *xyz = nullptr; float *rgba = nullptr;
-  cudaError_t e = cudaMalloc((void **)&flags, G);
-  if (!e) e = cudaMalloc((void **)&sel, G * 4);
+  FbDev<uint8_t> flags; FbDev<uint32_t> sel; FbDev<double> xyz; FbDev<float> rgba;
+  cudaError_t e = flags.alloc(G);
+  if (!e) e = sel.alloc(G);
   unsigned n = 0;
   if (!e) { k_vis_slice_flags<<<(unsigned)((G + 255) / 256), 256, 0, s>>>(g, cobs, slice, flags); e = vis_select(flags, G, sel, &n, s); }
   *count = n;
   const unsigned m = (long long)n < cap ? n : (unsigned)(cap < 0 ? 0 : cap);
   if (!e && m) {
-    e = cudaMalloc((void **)&xyz, (size_t)m * 24);
-    if (!e) e = cudaMalloc((void **)&rgba, (size_t)m * 16);
+    e = xyz.alloc((size_t)m * 3);
+    if (!e) e = rgba.alloc((size_t)m * 4);
     if (!e) {
       k_vis_slice_points<<<(m + 255) / 256, 256, 0, s>>>(g, cobs, sel, m, slice, max_dist, xyz, rgba);
       e = cudaMemcpyAsync(h_xyz, xyz, (size_t)m * 24, cudaMemcpyDeviceToHost, s);
@@ -120,6 +118,5 @@ cudaError_t fb_vis_slice(const FbGeom &g, const uint32_t *cobs, int slice, doubl
     }
     if (!e) e = cudaStreamSynchronize(s);
   }
-  cudaFree(flags); cudaFree(sel); cudaFree(xyz); cudaFree(rgba);
   return e;
 }

@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 
 from tests import scenes
-from tests.parity import compare
+from tests.parity import compare, invariants
 
 pytestmark = pytest.mark.gpu
 
@@ -245,6 +245,55 @@ def test_host_mirror_tracks_every_update(oracle_built, mode, cap, monkeypatch):
     assert d1 == d2 and tuple(g1) == tuple(g2)
     assert mir.GetDistance((9.0, 0.0, 0.0)) == -10000 and mir.GetDistWithGradTrilinear((9.0, 0.0, 0.0))[0] == -1
     mir.close()
+
+
+@pytest.mark.parametrize("mode", ["fast", "exact"])
+def test_two_occupancy_updates_before_esdf(oracle_built, mode):
+    """UpdateOccupancy twice, then one UpdateESDF: the insert / delete queues grow during the second call, and the pushes of the
+    first one must survive that growth.  A grown queue holds 1.5x what was asked for plus 1 MiB (2^18 entries), so the second
+    call pushes more than 2^18 crossings into each queue (EXACT), from every tile of the grid (FAST reserves 512 entries per
+    touched tile).  The many voxels it deletes become occupied through a lowered threshold, not through inserts, so that the
+    queues stay small until then."""
+    origin = (-6.4, -6.4, -3.2)
+    dev, ora = pair(oracle_built, mode, origin=origin, size=(12.8, 12.8, 6.4), params=scenes.PARAMS_DEFAULT)
+    gs = dev.grid_size                                                       # 128 x 128 x 64: 2048 tiles
+    allv = scenes.all_voxels(gs)
+    slab = allv[allv[:, 0] < 40]                                             # 640 tiles
+    rest = allv[allv[:, 0] >= 40]
+    rng = np.random.default_rng(12)
+    q = rest[rng.choice(np.flatnonzero(rest[:, 0] == 40), 50, replace=False)]
+    fresh = rest[rest[:, 0] > 40]
+    fresh = fresh[rng.permutation(len(fresh))]
+    lowered = (0.70, 0.35, 0.12, 0.97, 0.60)                                 # one hit (0.847) is occupied, one more miss (0.228) is not
+
+    def occupancy(vox, occ):
+        assert np.array_equal(dev.SetOccupancyBatchVox(vox, occ), ora.SetOccupancyBatchVox(vox, occ))
+        assert dev.UpdateOccupancy(True) == ora.UpdateOccupancy(True)
+
+    occupancy(slab, np.ones(len(slab), np.uint8))                            # one hit each: below the default threshold
+    for m in (dev, ora):
+        m.SetParameters(*lowered)                                            # the whole slab is occupied now, no queue push
+    occupancy(q, np.ones(len(q), np.uint8))                                  # 50 real obstacles next to the slab
+    dev.UpdateESDF(); ora.UpdateESDF()
+    occupancy(np.concatenate([q, fresh[:50]]), np.r_[np.zeros(50), np.ones(50)].astype(np.uint8))   # first call: 50 + 50
+    big = fresh[50:270050]
+    occupancy(np.concatenate([slab, big]), np.r_[np.zeros(len(slab)), np.ones(len(big))].astype(np.uint8))   # second call
+    dev.UpdateESDF(); ora.UpdateESDF()
+    sd, so = dev.stats(), ora.stats()
+    assert (sd["inserts"], sd["deletes"]) == (so["inserts"], so["deletes"]) == (len(big) + 50, len(slab) + 50)
+    if mode == "exact":
+        r = compare(dev, ora)
+        assert r["occ"] == 0 and r["dist"] == 0 and r["cobs_tie"] == 0 and r["cobs_nontie"] == 0, r
+        assert sd["expansions"] == so["expansions"]
+        pos = rng.uniform(-6.3, 6.2, (2000, 3)) * (1, 1, 0.5)
+        d1, g1 = dev.GetDistWithGradTrilinearBatch(pos)
+        d2, g2 = ora.GetDistWithGradTrilinearBatch(pos)
+        assert np.array_equal(d1, d2) and np.array_equal(g1, g2)
+    else:
+        r = compare(dev, ora, check_counters=True)
+        assert r["occ"] == 0 and r["counters"] == 0, r
+        inv = invariants(dev, np.log(0.6 / 0.4))
+        assert all(v == 0 for v in inv.values()), inv
 
 
 def test_occupancy_threshold_change_exact(oracle_built):
